@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ACR hot path (BASELINE.json metric: images/sec, 512x512, batch 256 per GPU).
 
-    python bench.py --gpus 1 --steps 10 --warmup 3
+    python bench.py --gpus 1 --steps 10 --warmup 3 [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's CPU implementation (oracle port)
@@ -200,7 +200,7 @@ def run_reference(args):
     a bounded sample of `ref_batch` frames of the batch-256 workload.  Rank 0 only."""
     if int(os.environ.get("RANK", "0")) != 0:
         return
-    steps, warm = max(1, min(args.steps, 5)), min(args.warmup, 1)
+    steps, warm = args.steps, min(args.warmup, 1)
     val, dt, cb = cpu_arm(args.ref_batch, steps, warm)
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": val, "unit": "images/s", "n_gpus": args.gpus, "steps": steps,
@@ -213,6 +213,34 @@ def run_reference(args):
 
 
 # -------------------------------------------------------------------------------- B200 arm
+DUMP_BYTES = 64 << 20
+# per-hand outputs of the parse kernels that fused_forward hands to its caller (top_idx / top_score / row_src are scratch)
+PARSE_OUTPUTS = ("params_pred", "cam", "global_orient", "hand_pose", "betas", "poses", "detection_flag", "reorganize_idx",
+                 "batch_ids", "centers_pred", "centers_conf", "hand_type", "offsets_out")
+
+
+def dump_outputs(dirname, bufs, mano, max_bytes=DUMP_BYTES):
+    """Write what one step returned to its caller as <dirname>/<name>.npy: the counts[2] valid rows of every parse and
+    MANO output (floats as float32, integers as float64, both exact) and the row counts.  Past `max_bytes` a fixed,
+    seeded subset of the rows is written; rows.npy names the rows written."""
+    import numpy as np
+    counts = bufs.counts.cpu().numpy()
+    n = int(counts[2])
+    arrays = {k: getattr(bufs, k)[:n] for k in PARSE_OUTPUTS}
+    arrays.update({k: v[:n] for k, v in mano.items()})
+    arrays = {k: v.cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: a.astype(np.float32 if a.dtype.kind == "f" else np.float64) for k, a in arrays.items()}
+    row_bytes = 8 + sum(a.itemsize * int(np.prod(a.shape[1:])) for a in arrays.values())   # 8: the entry of rows.npy
+    keep = (max_bytes - (64 << 10)) // row_bytes                                             # 64 KiB: counts + npy headers
+    rows = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    arrays = {k: a[rows] for k, a in arrays.items()}
+    arrays["rows"], arrays["counts"] = rows.astype(np.float64), counts.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, f"{k}.npy"), a)
+    return arrays
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -311,7 +339,14 @@ def run_b200(args):
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms_value, ms_per_rank = timed(lambda: step(frames_dev), args.steps)
+    last = {}
+
+    def value_step():
+        last["out"] = step(frames_dev)
+
+    ms_value, ms_per_rank = timed(value_step, args.steps)
+    if args.dump_outputs and rank == 0:        # before any later call re-uses the parse buffers
+        dump_outputs(args.dump_outputs, *last["out"])
 
     # ---- end to end: every step copies ITS frames from pinned host memory and reads ITS results back.
     # Two device staging buffers + a copy stream let the H2D of step i+1 overlap the kernels of step i
@@ -512,7 +547,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="cpu_baseline", action="store_false")
     ap.add_argument("--gather", default="fused", choices=["fused", "nccl"],
                     help="N>1: vertex all-gather fused into the MANO kernel (symmetric memory) or a separate NCCL call")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     if args.gpus > 1 or args.backbone != "hrnet_w32":
         args.cpu_baseline = False          # the CPU arm is the reference's own network (HRNet-W32)
     if args.impl == "reference":

@@ -135,6 +135,39 @@ def test_bench_traffic_stamp_and_thread_sweep(tmp_path, monkeypatch):
     assert best == 8 and list(sweep) == [8] and len(calls) == 2, (best, sweep, calls)   # warm-up + one timed run per candidate
 
 
+def test_bench_dump_outputs_writes_the_valid_rows(tmp_path):
+    """bench.py --dump-outputs: the counts[2] valid rows of every output as float32 / float64 .npy; past the byte budget the
+    same seeded subset of rows of every array, identical from run to run."""
+    sys.path.insert(0, ROOT)
+    import bench
+    from acr_b200.ops import ParseBuffers
+    B = 3
+    bufs = ParseBuffers(B, "cpu")
+    g = torch.Generator().manual_seed(0)
+    for k in bench.PARSE_OUTPUTS:
+        t = getattr(bufs, k)
+        t.copy_(torch.randn(t.shape, generator=g) if t.dtype.is_floating_point else torch.randint(0, 64, t.shape, generator=g))
+    bufs.counts[:3] = torch.tensor([2, 3, 5])
+    mano = {"verts": torch.randn(2 * B, 778, 3, generator=g), "joints": torch.randn(2 * B, 21, 3, generator=g)}
+    names = (*bench.PARSE_OUTPUTS, "verts", "joints")
+    src = {k: (mano[k] if k in mano else getattr(bufs, k))[:5].numpy() for k in names}
+    bench.dump_outputs(str(tmp_path / "all"), bufs, mano)
+    assert sorted(p.name for p in (tmp_path / "all").iterdir()) == sorted(f"{k}.npy" for k in names + ("rows", "counts"))
+    for k in names:
+        a = np.load(tmp_path / "all" / f"{k}.npy")
+        assert a.dtype in (np.float32, np.float64) and a.shape == src[k].shape and np.array_equal(a, src[k]), k
+    assert np.array_equal(np.load(tmp_path / "all" / "counts.npy"), bufs.counts.numpy())
+    budget = (64 << 10) + 45000                                  # room for 4 of the 5 rows (about 10.6 KB each)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), bufs, mano, max_bytes=budget)
+    rows = np.load(tmp_path / "a" / "rows.npy").astype(int)
+    assert len(rows) == 4 and np.array_equal(rows, np.unique(rows)) and rows.max() < 5
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= budget
+    for k in names:
+        a, b = np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "b" / f"{k}.npy")
+        assert np.array_equal(a, src[k][rows]) and np.array_equal(a, b), k
+
+
 def test_lazy_outputs_refuse_stale_maps():
     from acr.model import LazyOutputs
 
