@@ -58,7 +58,11 @@ _lib: Optional[C.CDLL] = None
 EXPORTS = ["acr_b200_last_error", "acr_b200_version", "acr_b200_mano_model_floats", "acr_b200_mano_pack_model",
            "acr_b200_mano_forward", "acr_b200_mano_forward_gather", "acr_b200_gather_wait", "acr_b200_cam_trans", "acr_b200_preprocess", "acr_b200_one_euro_state_floats", "acr_b200_one_euro_smooth", "acr_b200_rot6d_to_aa", "acr_b200_rodrigues", "acr_b200_parse",
            "acr_b200_plan_create", "acr_b200_plan_run", "acr_b200_plan_profile", "acr_b200_plan_num_launches", "acr_b200_plan_destroy",
-           "acr_b200_run_op", "acr_b200_pack_conv"]
+           "acr_b200_run_op", "acr_b200_conv_describe", "acr_b200_pack_conv"]
+
+# acr_b200_conv_describe: field order of its info array (ACR_CONV_INFO_* in include/acr_b200.h)
+CONV_INFO = ("ck", "mode", "b_resident", "nsplit", "nsub", "nbuf", "epilogue", "epi_nb", "SA", "SB", "grid", "vtiles")
+MODE_PATCH, MODE_RESIDENT, MODE_XPAIR, MODE_DIAG, MODE_P1, MODE_S2X = 1, 2, 4, 8, 16, 32
 
 
 def load() -> C.CDLL:
@@ -94,6 +98,7 @@ def load() -> C.CDLL:
     lib.acr_b200_plan_destroy.argtypes = [vp]
     lib.acr_b200_plan_destroy.restype = None
     lib.acr_b200_run_op.argtypes = [C.POINTER(Op), i32, vp, vp, vp, i32, vp]
+    lib.acr_b200_conv_describe.argtypes = [C.POINTER(Op), i32, vp, vp, i32, vp, i32]
     lib.acr_b200_pack_conv.argtypes = [vp] * 6 + [f32, i32, i32, i32, i32, i32, i32, vp, vp]
     _lib = lib
     return lib

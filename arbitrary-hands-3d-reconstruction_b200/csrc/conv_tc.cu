@@ -906,6 +906,14 @@ static int epi_staged_level() {
   return e ? atoi(e) : 1;
 }
 
+// ACR_B200_CONV_MAX_CTAS=n (read at plan creation, testing only): at most n persistent CTAs, so that small test
+// convs run several virtual tiles per CTA (TMEM buffer alternation, barrier phases and staging rings carried
+// across tiles, an odd grid for the N split).  Unset or <= 0: one CTA per SM.
+static int conv_max_ctas() {
+  const char* e = getenv("ACR_B200_CONV_MAX_CTAS");
+  return e ? atoi(e) : 0;
+}
+
 int conv_tc_prepare(const ConvArgs& a, int act_dtype, ConvTcPlan** out) {
   ACR_CHECK_ARG(a.out.H % TILE_Y == 0 && a.out.W % TILE_X == 0, "conv_tc: output %dx%d is not a multiple of the 16x16 super-tile", a.out.H, a.out.W);
   ACR_CHECK_ARG(a.in.pix_stride % 8 == 0 && a.cin_pad % 16 == 0 && a.cout_pad % 16 == 0 && a.cout_pad <= 1024,
@@ -1086,6 +1094,8 @@ int conv_tc_prepare(const ConvArgs& a, int act_dtype, ConvTcPlan** out) {
   p.SA = SA;
   pl->smem = fixed + p.b_region_bytes + (size_t)SA * p.a_stage_bytes;
   pl->grid = p.total_tiles * nsplit < num_sms() ? p.total_tiles * nsplit : num_sms();
+  const int cap = conv_max_ctas();
+  if (cap > 0 && pl->grid > cap) pl->grid = cap;
   *out = pl;
   return ACR_B200_OK;
 }
@@ -1110,36 +1120,49 @@ static int launch_inst(const ConvTcPlan* pl, cudaStream_t st) {
   return ACR_B200_OK;
 }
 
+// MODE bits of the kernel instance that runs a plan, or -1 (error set) when no instance exists for it
+static int plan_mode(const ConvTcPlan* pl) {
+  const ConvTcParams& p = pl->p;
+  const int mode = (p.patch_mode ? MODE_PATCH : 0) | (p.b_resident ? MODE_RESIDENT : 0);
+  if (pl->ck == 64 && p.s2x) {
+    if (p.debug) { set_error("conv_tc: no diagnostic instance of the x-paired stride-2 form"); return -1; }
+    return MODE_S2X | (p.b_resident ? MODE_RESIDENT : 0);
+  }
+  if (pl->ck == 64 && p.patch1) {
+    if (p.debug) { set_error("conv_tc: diagnostic instances exist for the three-box form only (ACR_B200_P1=0)"); return -1; }
+    if (p.xpair && !p.b_resident) { set_error("conv_tc: x-paired conv needs resident weights"); return -1; }
+    return mode | MODE_P1 | (p.xpair ? MODE_XPAIR : 0);
+  }
+  if (p.debug) {
+    if (pl->ck != 64 || mode != (MODE_PATCH | MODE_RESIDENT)) { set_error("conv_tc: diagnostic instances exist for CK=64 patch/resident only"); return -1; }
+    return mode | MODE_DIAG | (p.xpair ? MODE_XPAIR : 0);
+  }
+  if (pl->ck == 64 && p.xpair) {
+    if (mode != (MODE_PATCH | MODE_RESIDENT)) { set_error("conv_tc: x-paired conv needs resident weights"); return -1; }
+    return mode | MODE_XPAIR;
+  }
+  return mode;
+}
+
 template <int CK, typename T>
 static int launch_mode(const ConvTcPlan* pl, cudaStream_t st) {
-  const int mode = (pl->p.patch_mode ? MODE_PATCH : 0) | (pl->p.b_resident ? MODE_RESIDENT : 0);
-  if (CK == 64 && pl->p.s2x) {
-    if (pl->p.debug) { set_error("conv_tc: no diagnostic instance of the x-paired stride-2 form"); return ACR_B200_EINVAL; }
-    return pl->p.b_resident ? launch_inst<64, T, MODE_RESIDENT | MODE_S2X>(pl, st) : launch_inst<64, T, MODE_S2X>(pl, st);
-  }
-  if (CK == 64 && pl->p.patch1) {
-    if (pl->p.debug) { set_error("conv_tc: diagnostic instances exist for the three-box form only (ACR_B200_P1=0)"); return ACR_B200_EINVAL; }
-    if (pl->p.xpair) {
-      if (!pl->p.b_resident) { set_error("conv_tc: x-paired conv needs resident weights"); return ACR_B200_EINVAL; }
-      return launch_inst<64, T, MODE_PATCH | MODE_RESIDENT | MODE_XPAIR | MODE_P1>(pl, st);
-    }
-    return pl->p.b_resident ? launch_inst<64, T, MODE_PATCH | MODE_RESIDENT | MODE_P1>(pl, st)
-                            : launch_inst<64, T, MODE_PATCH | MODE_P1>(pl, st);
-  }
-  if (pl->p.debug) {
-    if (CK != 64 || mode != (MODE_PATCH | MODE_RESIDENT)) { set_error("conv_tc: diagnostic instances exist for CK=64 patch/resident only"); return ACR_B200_EINVAL; }
-    return pl->p.xpair ? launch_inst<64, T, MODE_PATCH | MODE_RESIDENT | MODE_XPAIR | MODE_DIAG>(pl, st)
-                       : launch_inst<64, T, MODE_PATCH | MODE_RESIDENT | MODE_DIAG>(pl, st);
-  }
-  if (CK == 64 && pl->p.xpair) {
-    if (mode != (MODE_PATCH | MODE_RESIDENT)) { set_error("conv_tc: x-paired conv needs resident weights"); return ACR_B200_EINVAL; }
-    return launch_inst<64, T, MODE_PATCH | MODE_RESIDENT | MODE_XPAIR>(pl, st);
-  }
-  switch (mode) {
+  constexpr int PR = MODE_PATCH | MODE_RESIDENT;
+  switch (plan_mode(pl)) {
+    case -1: return ACR_B200_EINVAL;
     case 0: return launch_inst<CK, T, 0>(pl, st);
-    case 1: return launch_inst<CK, T, 1>(pl, st);
-    case 2: return launch_inst<CK, T, 2>(pl, st);
-    default: return launch_inst<CK, T, 3>(pl, st);
+    case MODE_PATCH: return launch_inst<CK, T, MODE_PATCH>(pl, st);
+    case MODE_RESIDENT: return launch_inst<CK, T, MODE_RESIDENT>(pl, st);
+    case PR: return launch_inst<CK, T, PR>(pl, st);
+    // the remaining forms exist for CK = 64 only (plan_mode never picks them otherwise)
+    case MODE_S2X: return launch_inst<64, T, MODE_S2X>(pl, st);
+    case MODE_S2X | MODE_RESIDENT: return launch_inst<64, T, MODE_RESIDENT | MODE_S2X>(pl, st);
+    case MODE_PATCH | MODE_P1: return launch_inst<64, T, MODE_PATCH | MODE_P1>(pl, st);
+    case PR | MODE_P1: return launch_inst<64, T, PR | MODE_P1>(pl, st);
+    case PR | MODE_XPAIR | MODE_P1: return launch_inst<64, T, PR | MODE_XPAIR | MODE_P1>(pl, st);
+    case PR | MODE_XPAIR: return launch_inst<64, T, PR | MODE_XPAIR>(pl, st);
+    case PR | MODE_DIAG: return launch_inst<64, T, PR | MODE_DIAG>(pl, st);
+    case PR | MODE_XPAIR | MODE_DIAG: return launch_inst<64, T, PR | MODE_XPAIR | MODE_DIAG>(pl, st);
+    default: set_error("conv_tc: no kernel instance for MODE %d", plan_mode(pl)); return ACR_B200_EINVAL;
   }
 }
 
@@ -1150,6 +1173,27 @@ int conv_tc_launch(const ConvTcPlan* pl, cudaStream_t st) {
     case 32: return bf ? launch_mode<32, __nv_bfloat16>(pl, st) : launch_mode<32, __half>(pl, st);
     default: return bf ? launch_mode<16, __nv_bfloat16>(pl, st) : launch_mode<16, __half>(pl, st);
   }
+}
+
+int conv_tc_describe(const ConvTcPlan* pl, int32_t* info, int n_info) {
+  const int mode = plan_mode(pl);
+  if (mode < 0) return ACR_B200_EINVAL;
+  const ConvTcParams& p = pl->p;
+  int32_t v[ACR_CONV_INFO_N] = {};
+  v[ACR_CONV_INFO_CK] = pl->ck;
+  v[ACR_CONV_INFO_MODE] = mode;
+  v[ACR_CONV_INFO_B_RESIDENT] = p.b_resident;
+  v[ACR_CONV_INFO_NSPLIT] = p.nsplit;
+  v[ACR_CONV_INFO_NSUB] = p.nsub;
+  v[ACR_CONV_INFO_NBUF] = p.nbuf;
+  v[ACR_CONV_INFO_EPILOGUE] = p.tma_out ? 2 : (p.epi_staged ? 1 : 0);
+  v[ACR_CONV_INFO_EPI_NB] = p.epi_nb;
+  v[ACR_CONV_INFO_SA] = p.SA;
+  v[ACR_CONV_INFO_SB] = p.SB;
+  v[ACR_CONV_INFO_GRID] = pl->grid;
+  v[ACR_CONV_INFO_VTILES] = p.total_tiles * p.nsplit;
+  for (int i = 0; i < n_info && i < ACR_CONV_INFO_N; ++i) info[i] = v[i];
+  return ACR_B200_OK;
 }
 
 void conv_tc_free(ConvTcPlan* p) { delete p; }

@@ -75,6 +75,8 @@ int launch_pool_f32(const TensorRef& feat, const TensorRef& logits, float* part,
 struct ConvTcPlan;   // holds the TMA tensor maps of one conv op
 int conv_tc_prepare(const ConvArgs& a, int act_dtype, ConvTcPlan** out);
 int conv_tc_launch(const ConvTcPlan* p, cudaStream_t st);
+// the plan's kernel instance and schedule as the ACR_CONV_INFO_* fields of include/acr_b200.h (first n_info of them)
+int conv_tc_describe(const ConvTcPlan* p, int32_t* info, int n_info);
 void conv_tc_free(ConvTcPlan* p);
 
 }  // namespace acr

@@ -330,6 +330,22 @@ extern "C" int acr_b200_run_op(const acr_b200_op* op, int batch, void* arena, co
                  static_cast<const char*>(external), act_dtype, nullptr, static_cast<cudaStream_t>(stream));
 }
 
+extern "C" int acr_b200_conv_describe(const acr_b200_op* op, int batch, void* arena, const void* weights,
+                                      int act_dtype, int32_t* info, int n_info) {
+  ACR_CHECK_ARG(op && batch > 0 && arena && weights && (info || n_info == 0), "conv_describe: bad arguments");
+  ACR_CHECK_ARG(op->kind == ACR_OP_CONV && (act_dtype == ACR_DT_BF16 || act_dtype == ACR_DT_F16),
+                "conv_describe: a tensor-core conv (ACR_OP_CONV, bf16 / f16) has no plan to describe otherwise");
+  ConvArgs a;
+  int rc = make_conv_args(*op, batch, static_cast<char*>(arena), static_cast<const char*>(weights), nullptr, &a);
+  if (rc) return rc;
+  ConvTcPlan* pl = nullptr;
+  rc = conv_tc_prepare(a, act_dtype, &pl);
+  if (rc) return rc;
+  rc = conv_tc_describe(pl, info, n_info);
+  conv_tc_free(pl);
+  return rc;
+}
+
 // BN folding + repack, host side.  y = gamma*(conv(x)+cb-mean)/sqrt(var+eps)+beta = conv'(x) + b'
 extern "C" int acr_b200_pack_conv(const float* w, const float* conv_bias, const float* g, const float* beta,
                                   const float* mean, const float* var, float eps, int cout, int cin, int k,

@@ -280,6 +280,28 @@ void acr_b200_plan_destroy(acr_b200_plan* plan);
 int acr_b200_run_op(const acr_b200_op* op, int batch, void* arena, const void* weights,
                     const void* external, int act_dtype, void* stream);
 
+/* Which kernel instance and schedule an ACR_OP_CONV launch gets (tests: proves what a case exercised).
+ * Builds the conv's plan exactly as plan_create / run_op do (same environment switches), writes the first
+ * n_info of the fields below to `info` (host) and frees the plan; nothing is launched.  Encoding the TMA
+ * tensor maps needs the CUDA driver, so this fails on a machine without one.
+ *   CK          channel chunk of the K loop (16 / 32 / 64)
+ *   MODE        template bits of the instance: 1 PATCH, 2 RESIDENT, 4 XPAIR, 8 DIAG, 16 P1, 32 S2X
+ *   B_RESIDENT  weights resident in shared memory for the whole kernel
+ *   NSPLIT/NSUB each 16x16 super-tile is NSPLIT virtual tiles of NSUB output channels
+ *   NBUF        TMEM accumulator buffers (2 = the epilogue of one tile overlaps the MMAs of the next)
+ *   EPILOGUE    0 direct stores, 1 staged (per-warp slabs, TMA residual loads + TMA stores), 2 TMA store
+ *   EPI_NB      slab buffers per epilogue warp of the staged epilogue
+ *   SA/SB       A / B operand stages (SB = 0: resident weights)
+ *   GRID        persistent CTAs = min(VTILES, SMs, ACR_B200_CONV_MAX_CTAS if set)
+ *   VTILES      virtual tiles of the launch (super-tiles of all images x NSPLIT)                  */
+enum {
+  ACR_CONV_INFO_CK, ACR_CONV_INFO_MODE, ACR_CONV_INFO_B_RESIDENT, ACR_CONV_INFO_NSPLIT, ACR_CONV_INFO_NSUB,
+  ACR_CONV_INFO_NBUF, ACR_CONV_INFO_EPILOGUE, ACR_CONV_INFO_EPI_NB, ACR_CONV_INFO_SA, ACR_CONV_INFO_SB,
+  ACR_CONV_INFO_GRID, ACR_CONV_INFO_VTILES, ACR_CONV_INFO_N
+};
+int acr_b200_conv_describe(const acr_b200_op* op, int batch, void* arena, const void* weights,
+                           int act_dtype, int32_t* info, int n_info);
+
 /* Host-side weight folding/packing for one conv (acr_b200_weights_pack of SURVEY.md 8b):
  * folds eval-mode BatchNorm (acr/model.py BN after every conv) into w/b and repacks
  * OIHW fp32 -> [cout_pad][kh][kw][cin_pad] 16-bit (K-major rows for the UMMA B operand).

@@ -84,6 +84,7 @@ def run_conv_case(kind, B, H, W, cin, cout, k, s, relu, residual, bias, bn, out_
     oesz = 4 if out_f32 else 2
     obytes = B * Ho * Wo * cout_pad * oesz
     arena = torch.zeros(off_o + obytes + 1024, dtype=torch.uint8)
+    arena[off_o: off_o + obytes] = 0xFF      # NaN: a channel the kernel does not write (pad channels included) stays NaN
     arena[off_x: off_x + xin.numel() * esz] = xin.view(torch.uint8).flatten()
     if residual:
         rin = to_nhwc_padded(res, res_stride, tdt)
