@@ -64,9 +64,12 @@ class ACR(nn.Module):
         parse buffers are shared per batch size, consume them before the next call).  ``peers``
         (acr_b200.dist.PeerVertexGather): the MANO kernel also stores vertices and row counts into every
         rank's gather buffer."""
-        B = images_rgb_u8.shape[0]
         meta = {'image': images_rgb_u8, 'offsets': offsets, 'batch_ids': None}
         eng, bufs = self.model.forward_dense(meta)
+        return bufs, self._mano_dense(bufs, peers)
+
+    def _mano_dense(self, bufs, peers=None):
+        """MANO (+ cam_trans) over the 2B rows of dense parse buffers; rows >= counts[2] are skipped on the device."""
         from acr_b200 import ops as _ops
         ml, mr = self.mano_regression.models()
         mano = _ops.mano_forward(ml, mr, bufs.poses, bufs.betas, bufs.hand_type, 1, self.mano_regression.center_idx,
@@ -74,36 +77,70 @@ class ACR(nn.Module):
         if args().cam_trans_mode == 'lstsq':
             mano['cam_trans'] = _ops.cam_trans(mano['joints'], mano['pj2d'], args().focal_length, 512.0,
                                                n_dev=bufs.counts[2:3])
-        return bufs, mano
+        return mano
 
     @torch.no_grad()
-    def capture_graph(self, batch: int, device=None):
+    def stream_forward(self, images_rgb_u8, offsets, streams=None, stream_ids=None):
+        """B frames of B independent video streams in one sync-free pass: backbone + heads, per-frame parse (every
+        frame parsed as the reference parses it alone; row b = left hand of frame b, row B + b = its right hand,
+        all 2B rows valid), then -- when ``streams`` (acr_b200.ops.StreamStates) is given -- OneEuro smoothing with
+        ``smooth_coeff``, each frame with its own stream's filters, then MANO over the 2B rows and cam_trans.
+        ``stream_ids``: stream of each slot (int32, length B; -1 = padding slot, not smoothed); None = slot b is
+        stream b.  Host ids are validated (distinct, below n_streams); a CUDA int32 tensor is used as is.  Returns
+        ``(bufs, mano)`` with fused_forward's zero-copy contract."""
+        from acr_b200 import ops as _ops
+        B = images_rgb_u8.shape[0]
+        if streams is not None:      # validate before any launch
+            ids = _ops.check_stream_ids(stream_ids, B, streams.n_streams)
+        meta = {'image': images_rgb_u8, 'offsets': offsets, 'batch_ids': None}
+        eng, bufs = self.model.forward_dense(meta, per_frame=True)
+        if streams is not None:
+            _ops.one_euro_smooth_streams(bufs.poses, bufs.betas, streams, ids.to(bufs.poses.device),
+                                         hand_type=bufs.hand_type, detection_flag=bufs.detection_flag,
+                                         batch_ids=bufs.batch_ids, smooth_coeff=float(self.smooth_coeff))
+        return bufs, self._mano_dense(bufs)
+
+    @torch.no_grad()
+    def capture_graph(self, batch: int, device=None, streams=None):
         """CUDA-graph the whole sync-free pipeline (backbone + heads + parse + MANO + cam_trans, ~380 kernel
         launches) for a fixed batch size: returns ``replay(frames_u8, offsets) -> (bufs, mano)`` that copies
         the inputs into static buffers and launches ONE graph.  This is what makes the reference's
         frame-by-frame video / webcam loop (acr/main.py:183-201, batch 1) latency-bound by the GPU instead
-        of by ~380 host-side launches."""
+        of by ~380 host-side launches.  ``streams`` (acr_b200.ops.StreamStates): the graph is stream_forward
+        instead (per-frame parse + per-stream smoothing, state on the device), and
+        ``replay(frames_u8, offsets, stream_ids=None)`` also copies the slot -> stream ids (None: slot b is stream
+        b) into a static buffer."""
+        from acr_b200 import ops as _ops
         dev = torch.device(device) if device is not None else next(self.model.parameters()).device
         frames = torch.zeros(batch, args().input_size, args().input_size, 3, dtype=torch.uint8, device=dev)
         offsets = torch.zeros(batch, 10, device=dev)
+        if streams is None:
+            run = lambda: self.fused_forward(frames, offsets)
+        else:
+            ids = torch.full((batch,), -1, dtype=torch.int32, device=dev)     # warm-up: padding only, no state touched
+            run = lambda: self.stream_forward(frames, offsets, streams, ids)
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):                       # warm-up: builds the engine, sets func attributes
             for _ in range(2):
-                self.fused_forward(frames, offsets)
+                run()
         torch.cuda.current_stream(dev).wait_stream(side)
         torch.cuda.synchronize(dev)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            bufs, mano = self.fused_forward(frames, offsets)
+            bufs, mano = run()
 
-        def replay(frames_u8, offs):
+        def replay(frames_u8, offs, stream_ids=None):
             frames.copy_(frames_u8, non_blocking=True)
             offsets.copy_(offs, non_blocking=True)
+            if streams is not None:
+                ids.copy_(_ops.check_stream_ids(stream_ids, batch, streams.n_streams))
+            elif stream_ids is not None:
+                raise ValueError("stream_ids needs a graph captured with streams=")
             graph.replay()
             return bufs, mano
 
-        replay.graph, replay.static_inputs = graph, (frames, offsets)
+        replay.graph, replay.static_inputs = graph, (frames, offsets) if streams is None else (frames, offsets, ids)
         return replay
 
     @torch.no_grad()

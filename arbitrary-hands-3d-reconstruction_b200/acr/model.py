@@ -175,15 +175,16 @@ class ACR(nn.Module):
         return outputs
 
     @torch.no_grad()
-    def forward_dense(self, meta_data):
+    def forward_dense(self, meta_data, per_frame=False):
         """Sync-free variant for the fused pipeline: runs backbone + heads + parse and returns the
         engine and the worst-case (2B rows) parse buffers; row validity lives in ``bufs.counts``.
+        ``per_frame``: every image parsed as a batch of one, rows b / B + b = left / right hand of image b.
         ZERO COPY: the returned buffers are the per-batch-size cached ones and alias the next call's
         results -- consume (or copy) them before the next forward of the same batch size."""
         img, dev = self._image(meta_data)
         eng = self.engine(img.shape[0], dev)
         eng.run(img)
-        bufs = self._result_parser.launch(eng.parse_inputs(), img.shape[0], meta_data, dev)
+        bufs = self._result_parser.launch(eng.parse_inputs(), img.shape[0], meta_data, dev, per_frame=per_frame)
         return eng, bufs
 
     @torch.no_grad()

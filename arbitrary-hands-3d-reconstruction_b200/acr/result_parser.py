@@ -28,19 +28,20 @@ class ResultParser(nn.Module):
                              "(the reference's shipped configuration) are supported")
         self._pbufs = {}
 
-    def _parse_buffers(self, B, device):
-        key = (B, str(device))
+    def _parse_buffers(self, B, device, per_frame=False):
+        key = (B, str(device), per_frame)
         if key not in self._pbufs:
             self._pbufs[key] = _ops.ParseBuffers(B, device)
         return self._pbufs[key]
 
     # ------------------------------------------------------------------ kernels
-    def launch(self, maps, B, meta_data, device):
-        """Enqueue the parse kernels; returns the worst-case buffers (no sync)."""
-        bufs = self._parse_buffers(B, device)
+    def launch(self, maps, B, meta_data, device, per_frame=False):
+        """Enqueue the parse kernels; returns the worst-case buffers (no sync).  ``per_frame``: each image parsed
+        as a batch of one into fixed rows (independent video streams), see acr_b200.ops.parse_maps."""
+        bufs = self._parse_buffers(B, device, per_frame)
         ids = meta_data.get('batch_ids') if meta_data is not None else None
         offs = meta_data.get('offsets') if meta_data is not None else None
-        _ops.parse_maps(maps, B, bufs, ids, offs, args().centermap_conf_thresh)
+        _ops.parse_maps(maps, B, bufs, ids, offs, args().centermap_conf_thresh, per_frame=per_frame)
         return bufs
 
     @staticmethod

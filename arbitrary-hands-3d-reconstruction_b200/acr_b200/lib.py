@@ -56,7 +56,9 @@ class Gather(C.Structure):
 _lib: Optional[C.CDLL] = None
 
 EXPORTS = ["acr_b200_last_error", "acr_b200_version", "acr_b200_mano_model_floats", "acr_b200_mano_pack_model",
-           "acr_b200_mano_forward", "acr_b200_mano_forward_gather", "acr_b200_gather_wait", "acr_b200_cam_trans", "acr_b200_preprocess", "acr_b200_one_euro_state_floats", "acr_b200_one_euro_smooth", "acr_b200_rot6d_to_aa", "acr_b200_rodrigues", "acr_b200_parse",
+           "acr_b200_mano_forward", "acr_b200_mano_forward_gather", "acr_b200_gather_wait", "acr_b200_cam_trans", "acr_b200_preprocess", "acr_b200_one_euro_state_floats", "acr_b200_one_euro_smooth",
+           "acr_b200_one_euro_smooth_streams", "acr_b200_rot6d_to_aa", "acr_b200_rodrigues", "acr_b200_parse",
+           "acr_b200_parse_per_frame",
            "acr_b200_plan_create", "acr_b200_plan_run", "acr_b200_plan_profile", "acr_b200_plan_num_launches", "acr_b200_plan_destroy",
            "acr_b200_run_op", "acr_b200_conv_describe", "acr_b200_pack_conv"]
 
@@ -87,9 +89,11 @@ def load() -> C.CDLL:
     lib.acr_b200_preprocess.argtypes = [vp, i32, i32, i32, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp]
     lib.acr_b200_one_euro_state_floats.restype = C.c_size_t
     lib.acr_b200_one_euro_smooth.argtypes = [vp, vp, vp, vp, vp, i32, vp, f32, vp]
+    lib.acr_b200_one_euro_smooth_streams.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp, i32, vp, f32, vp]
     lib.acr_b200_rot6d_to_aa.argtypes = [vp, i32, vp, vp]
     lib.acr_b200_rodrigues.argtypes = [vp, i32, vp, vp]
     lib.acr_b200_parse.argtypes = [Map] * 6 + [i32, f32, vp, vp, ParseOut, vp]
+    lib.acr_b200_parse_per_frame.argtypes = [Map] * 6 + [i32, f32, vp, vp, ParseOut, vp]
     lib.acr_b200_plan_create.argtypes = [C.POINTER(Op), i32, i32, vp, C.c_size_t, vp, C.c_size_t, i32,
                                          C.POINTER(vp)]
     lib.acr_b200_plan_run.argtypes = [vp, vp, vp]

@@ -109,6 +109,78 @@ def one_euro_smooth(poses: torch.Tensor, betas: torch.Tensor, state: OneEuroStat
                                                       L.current_stream(dev)), "one_euro_smooth")
 
 
+class StreamStates:
+    """Device-side filter history of ``n_streams`` independent video streams (acr_b200_one_euro_smooth_streams):
+    one OneEuroState-sized block per stream, zero = no history."""
+
+    def __init__(self, n_streams: int, device):
+        if int(n_streams) < 1:
+            raise ValueError("StreamStates needs at least one stream")
+        self.n_streams = int(n_streams)
+        self.block = int(L.load().acr_b200_one_euro_state_floats())
+        self.state = torch.zeros(self.n_streams * self.block, device=device)
+
+    def reset(self, ids=None) -> None:
+        """Forget the history of streams ``ids`` (all when None), e.g. when a stream starts a new clip.
+        Enqueued on the current stream: launches already enqueued still see the old history."""
+        if ids is None:
+            self.state.zero_()
+            return
+        ids = torch.as_tensor(ids, dtype=torch.int64).reshape(-1)
+        if ids.numel() and (int(ids.min()) < 0 or int(ids.max()) >= self.n_streams):
+            raise ValueError(f"stream ids must lie in [0, {self.n_streams})")
+        self.state.view(self.n_streams, self.block).index_fill_(0, ids.to(self.state.device), 0.0)
+
+
+def check_stream_ids(stream_ids, n_slots: Optional[int], n_streams: int) -> torch.Tensor:
+    """Slot -> stream map of one batch: int32, one id per slot, a negative id (-1) for a padding slot, the others
+    distinct and below ``n_streams``.  None = slot b is stream b.  Ids from the host (list, numpy, CPU tensor) are
+    validated and returned as a CPU int32 tensor; a CUDA int32 tensor is returned as is, only its shape checked
+    (its values stay on the device: ids outside [0, n_streams) are padding, distinct ones are the caller's duty)."""
+    if stream_ids is None:
+        if n_slots is None:
+            raise ValueError("stream ids are required")
+        stream_ids = torch.arange(n_slots, dtype=torch.int32)
+    if isinstance(stream_ids, torch.Tensor) and stream_ids.is_cuda:
+        if stream_ids.dtype != torch.int32 or stream_ids.dim() != 1 or \
+                (n_slots is not None and stream_ids.numel() != n_slots):
+            raise ValueError(f"device stream ids must be a 1-D int32 tensor with one id per slot ({n_slots})")
+        return stream_ids.contiguous()
+    ids = torch.as_tensor(stream_ids)
+    if ids.dtype.is_floating_point or ids.dtype.is_complex or ids.dtype == torch.bool:
+        raise TypeError(f"stream ids must be integers, got {ids.dtype}")
+    if ids.dim() != 1 or (n_slots is not None and ids.numel() != n_slots):
+        raise ValueError(f"stream ids: expected one id per slot ({n_slots}), got shape {tuple(ids.shape)}")
+    if ids.numel() and (int(ids.min()) < -2 ** 31 or int(ids.max()) >= 2 ** 31):
+        raise ValueError("stream ids must fit in int32")
+    live = ids[ids >= 0]
+    if live.numel() and int(live.max()) >= n_streams:
+        raise ValueError(f"stream id {int(live.max())} is not below n_streams = {n_streams}")
+    if live.unique().numel() != live.numel():
+        raise ValueError("stream ids must be distinct within one batch (two slots of one stream would race on its "
+                         "filter state)")
+    return ids.to(torch.int32).cpu().contiguous()
+
+
+def one_euro_smooth_streams(poses: torch.Tensor, betas: torch.Tensor, states: StreamStates, stream_ids,
+                            hand_type: torch.Tensor, detection_flag: Optional[torch.Tensor], batch_ids: torch.Tensor,
+                            smooth_coeff: float = 4.0, n_dev: Optional[torch.Tensor] = None) -> None:
+    """In-place temporal smoothing of (n,48) poses and (n,10) betas, row r with the filter bank of stream
+    ``stream_ids[batch_ids[r]]`` and hand ``hand_type[r]`` (the reference's per-frame filters of acr/main.py:69-83,
+    one pair per stream).  ``stream_ids`` as in check_stream_ids: host ids are validated, a CUDA tensor is not."""
+    ids = check_stream_ids(stream_ids, None, states.n_streams).to(poses.device)
+    dev = L.require_cuda(poses, betas, hand_type, detection_flag, batch_ids, n_dev, ids, states.state)
+    assert poses.is_contiguous() and betas.is_contiguous() and poses.dtype == betas.dtype == torch.float32
+    hand_type = hand_type.contiguous().to(torch.int32)
+    batch_ids = batch_ids.contiguous().to(torch.int64)
+    if poses.shape[0]:
+        with L.on(dev):
+            L.check(L.load().acr_b200_one_euro_smooth_streams(
+                L.ptr(poses), L.ptr(betas), L.ptr(hand_type), L.ptr(detection_flag), L.ptr(batch_ids), L.ptr(ids),
+                states.n_streams, L.ptr(n_dev), poses.shape[0], L.ptr(states.state), float(smooth_coeff),
+                L.current_stream(dev)), "one_euro_smooth_streams")
+
+
 # ------------------------------------------------------------------------------ rotations
 def rot6d_to_aa(rot6d: torch.Tensor) -> torch.Tensor:
     """(N, 6*J) -> (N, 3*J); drop-in for acr.utils.rot6D_to_angular."""
@@ -158,9 +230,11 @@ class ParseBuffers:
 
 
 def parse_maps(maps: Dict[str, tuple], B: int, bufs: ParseBuffers, meta_batch_ids: Optional[torch.Tensor],
-               offsets: Optional[torch.Tensor], conf_thresh: float = 0.35) -> None:
+               offsets: Optional[torch.Tensor], conf_thresh: float = 0.35, per_frame: bool = False) -> None:
     """maps[name] = (fp32 CUDA tensor in NHWC layout, pix_stride) for l/r_center, l/r_params, l/r_prior.
-    Fills ``bufs`` asynchronously on the current stream (no host sync)."""
+    Fills ``bufs`` asynchronously on the current stream (no host sync).  ``per_frame``: every image parsed as a
+    batch of one, fixed rows (b = left hand of image b, B + b = its right hand; acr_b200_parse_per_frame) instead
+    of the reference's batch parse with its batch-wide rules (acr_b200_parse)."""
     lib = L.load()
     ms = []
     dev = L.require_cuda(bufs.counts, *[maps[k][0] for k in maps])
@@ -175,8 +249,8 @@ def parse_maps(maps: Dict[str, tuple], B: int, bufs: ParseBuffers, meta_batch_id
     if offsets is not None:
         offsets = offsets.to(device=bufs.counts.device, dtype=torch.float32).contiguous()
     with L.on(dev):
-        rc = lib.acr_b200_parse(*ms, B, float(conf_thresh), L.ptr(meta_batch_ids), L.ptr(offsets), bufs.struct(),
-                                L.current_stream(dev))
+        fn = lib.acr_b200_parse_per_frame if per_frame else lib.acr_b200_parse
+        rc = fn(*ms, B, float(conf_thresh), L.ptr(meta_batch_ids), L.ptr(offsets), bufs.struct(), L.current_stream(dev))
     L.check(rc, "parse")
     # keep the inputs alive until the kernels have run
     bufs._keep = (meta_batch_ids, offsets, [m for m in maps.values()])

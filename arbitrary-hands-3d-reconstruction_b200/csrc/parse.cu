@@ -11,6 +11,9 @@
 //   2. parse_scan   1 CTA: stable compaction "left hands of all images, then right hands", the
 //                   dummy-row rule for a side with no detection, the batch-global determine_coeff
 //                   decision, counts.
+//      parse_slot   (acr_b200_parse_per_frame instead of parse_scan) one thread per image: the
+//                   fixed layout "row b = left hand of image b, row B+b = its right hand", each
+//                   image parsed as the reference parses a batch of one.
 //   3. parse_gather grid (2B): per output row gather 109 params at the centre (+106 prior values
 //                   read at the OTHER hand's centre), split, 16 x rot6d->axis-angle.
 #include "common.cuh"
@@ -28,8 +31,20 @@ struct ParseParams {
   const int64_t* meta_ids;
   const float* offsets;
   acr_b200_parse_out o;
-  int32_t* row_src;  // (2B,4): image, side, flat index, other side's flat index (or -1)
+  int32_t* row_src;  // (2B,4): image, side word, flat index, other side's flat index (or -1)
 };
+
+// side word of row_src: bit 0 = side; ROW_DUMMY marks a per-frame dummy row (its image has no detection on
+// that side).  parse_scan never sets it: its dummy rows are recognised by the side's batch-wide count of 0.
+constexpr int ROW_DUMMY = 2;
+
+// determine_coeff (result_parser.py:42-47) on two flat centre indices: the cross-hand prior is kept iff the
+// centres are at most 32 apart on the 64-grid ([y,x] distance in fp32, like the reference).
+__device__ __forceinline__ bool centres_near(int il, int ir) {
+  const float dy = (float)(il >> 6) - (float)(ir >> 6), dx = (float)(il & 63) - (float)(ir & 63);
+  const float d = sqrtf(dy * dy + dx * dx);
+  return !(d > 32.f);
+}
 
 __global__ void __launch_bounds__(256) parse_top1_kernel(ParseParams p) {
   __shared__ float s_map[NPIX];
@@ -114,12 +129,7 @@ __global__ void __launch_bounds__(1024) parse_scan_kernel(ParseParams p) {
   __syncthreads();
   // determine_coeff: distance between the first left and the first right centre of the batch
   bool prior_on = false;
-  if (nl > 0 && nr > 0) {
-    const int il = p.o.top_idx[s_first[0] * 2 + 0], ir = p.o.top_idx[s_first[1] * 2 + 1];
-    const float dy = (float)(il >> 6) - (float)(ir >> 6), dx = (float)(il & 63) - (float)(ir & 63);
-    const float d = sqrtf(dy * dy + dx * dx);
-    prior_on = !(d > 32.f);
-  }
+  if (nl > 0 && nr > 0) prior_on = centres_near(p.o.top_idx[s_first[0] * 2 + 0], p.o.top_idx[s_first[1] * 2 + 1]);
   int pos[2] = {s_cnt[0][t] - c[0], s_cnt[1][t] - c[1]};  // exclusive prefix
   for (int i = 0; i < per; ++i) {
     const int b = t * per + i;
@@ -144,14 +154,39 @@ __global__ void __launch_bounds__(1024) parse_scan_kernel(ParseParams p) {
   }
 }
 
+// Per-frame rows: image b alone is a batch of one for the reference, so a side it did not detect gets that
+// batch's dummy row (pixel 0 of image b, no prior) and the prior is decided on image b's own pair.
+// counts[3..5] are accumulated with atomics: the caller zeroes `counts` before the launch.
+__global__ void __launch_bounds__(128) parse_slot_kernel(ParseParams p) {
+  const int B = p.B, b = blockIdx.x * blockDim.x + threadIdx.x;
+  bool dl = false, dr = false;
+  if (b < B) {
+    dl = p.o.top_score[b * 2 + 0] > p.thresh;
+    dr = p.o.top_score[b * 2 + 1] > p.thresh;
+    const int il = p.o.top_idx[b * 2 + 0], ir = p.o.top_idx[b * 2 + 1];
+    const bool prior_on = dl && dr && centres_near(il, ir);
+    int32_t* r = p.row_src + (size_t)b * 4;
+    r[0] = b; r[1] = dl ? 0 : ROW_DUMMY; r[2] = dl ? il : 0; r[3] = prior_on ? ir : -1;
+    r = p.row_src + (size_t)(B + b) * 4;
+    r[0] = b; r[1] = dr ? 1 : 1 | ROW_DUMMY; r[2] = dr ? ir : 0; r[3] = prior_on ? il : -1;
+  }
+  const int nl = __popc(__ballot_sync(0xffffffffu, dl)), nr = __popc(__ballot_sync(0xffffffffu, dr));
+  if ((threadIdx.x & 31) == 0 && (nl | nr)) {
+    atomicAdd(&p.o.counts[3], nl + nr);
+    atomicAdd(&p.o.counts[4], nl);
+    atomicAdd(&p.o.counts[5], nr);
+  }
+  if (b == 0) { p.o.counts[0] = B; p.o.counts[1] = B; p.o.counts[2] = 2 * B; }
+}
+
 __global__ void __launch_bounds__(128) parse_gather_kernel(ParseParams p) {
   __shared__ float s_p[112];
   const int r = blockIdx.x, t = threadIdx.x;
   const int N = p.o.counts[2];
   if (r >= N) return;
   const int32_t* rs = p.row_src + (size_t)r * 4;
-  const int b = rs[0], side = rs[1], fi = rs[2], ofi = rs[3];
-  const bool real = side == 0 ? (p.o.counts[4] > 0) : (p.o.counts[5] > 0);
+  const int b = rs[0], side = rs[1] & 1, fi = rs[2], ofi = rs[3];
+  const bool real = !(rs[1] & ROW_DUMMY) && (side == 0 ? (p.o.counts[4] > 0) : (p.o.counts[5] > 0));
   if (t < 109) {
     const acr_b200_map pm = p.params[side];
     float v = pm.ptr[((size_t)b * NPIX + fi) * pm.pix_stride + t];
@@ -193,10 +228,10 @@ __global__ void __launch_bounds__(128) parse_gather_kernel(ParseParams p) {
 
 using namespace acr;
 
-extern "C" int acr_b200_parse(acr_b200_map l_center, acr_b200_map r_center, acr_b200_map l_params,
-                              acr_b200_map r_params, acr_b200_map l_prior, acr_b200_map r_prior, int B,
-                              float conf_thresh, const int64_t* meta_batch_ids, const float* offsets,
-                              acr_b200_parse_out out, void* stream) {
+static int parse_launch(acr_b200_map l_center, acr_b200_map r_center, acr_b200_map l_params, acr_b200_map r_params,
+                        acr_b200_map l_prior, acr_b200_map r_prior, int B, float conf_thresh,
+                        const int64_t* meta_batch_ids, const float* offsets, acr_b200_parse_out out, bool per_frame,
+                        cudaStream_t st) {
   ACR_CHECK_ARG(B > 0, "parse: B must be positive");
   ACR_CHECK_ARG(l_center.ptr && r_center.ptr && l_params.ptr && r_params.ptr && l_prior.ptr && r_prior.ptr,
                 "parse: null map");
@@ -210,12 +245,32 @@ extern "C" int acr_b200_parse(acr_b200_map l_center, acr_b200_map r_center, acr_
   p.prior[0] = l_prior; p.prior[1] = r_prior;
   p.B = B; p.thresh = conf_thresh; p.meta_ids = meta_batch_ids; p.offsets = offsets; p.o = out;
   p.row_src = out.row_src;
-  cudaStream_t st = (cudaStream_t)stream;
   parse_top1_kernel<<<dim3(B, 2), 256, 0, st>>>(p);
   ACR_CHECK_LAUNCH();
-  parse_scan_kernel<<<1, 1024, 0, st>>>(p);
+  if (per_frame) {
+    ACR_CHECK_CUDA(cudaMemsetAsync(out.counts, 0, 8 * sizeof(int32_t), st));
+    parse_slot_kernel<<<(B + 127) / 128, 128, 0, st>>>(p);
+  } else {
+    parse_scan_kernel<<<1, 1024, 0, st>>>(p);
+  }
   ACR_CHECK_LAUNCH();
   parse_gather_kernel<<<2 * B, 128, 0, st>>>(p);
   ACR_CHECK_LAUNCH();
   return ACR_B200_OK;
+}
+
+extern "C" int acr_b200_parse(acr_b200_map l_center, acr_b200_map r_center, acr_b200_map l_params,
+                              acr_b200_map r_params, acr_b200_map l_prior, acr_b200_map r_prior, int B,
+                              float conf_thresh, const int64_t* meta_batch_ids, const float* offsets,
+                              acr_b200_parse_out out, void* stream) {
+  return parse_launch(l_center, r_center, l_params, r_params, l_prior, r_prior, B, conf_thresh, meta_batch_ids,
+                      offsets, out, false, (cudaStream_t)stream);
+}
+
+extern "C" int acr_b200_parse_per_frame(acr_b200_map l_center, acr_b200_map r_center, acr_b200_map l_params,
+                                        acr_b200_map r_params, acr_b200_map l_prior, acr_b200_map r_prior, int B,
+                                        float conf_thresh, const int64_t* meta_batch_ids, const float* offsets,
+                                        acr_b200_parse_out out, void* stream) {
+  return parse_launch(l_center, r_center, l_params, r_params, l_prior, r_prior, B, conf_thresh, meta_batch_ids,
+                      offsets, out, true, (cudaStream_t)stream);
 }

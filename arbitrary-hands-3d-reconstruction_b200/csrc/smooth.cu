@@ -8,6 +8,8 @@
 //   x_hat = lowpass(x, alpha(mincutoff + beta*|lowpass(dx, alpha(dcutoff))|)),  dx = (x - x_prev)*freq,
 //   alpha(c) = 1 / (1 + (1/(2 pi c)) / (1/freq)),  freq = 30, beta = 0.7, dcutoff = 1,
 //   mincutoff = smooth_coeff (pose, root rotation) | 0.6 (betas).
+// Many streams: the state is one block of two banks per stream; a row's bank is (stream_ids[batch_ids[row]],
+// hand type).  Without stream ids there is one stream and the bank is the hand type alone.
 #include "common.cuh"
 #include "rotation.cuh"
 
@@ -25,6 +27,8 @@ __device__ __forceinline__ float one_euro_alpha(float cutoff) {
 __global__ void __launch_bounds__(SM_ELEMS) one_euro_kernel(float* __restrict__ poses, float* __restrict__ betas,
                                                             const int32_t* __restrict__ hand_type,
                                                             const float* __restrict__ detection_flag,
+                                                            const int64_t* __restrict__ batch_ids,
+                                                            const int32_t* __restrict__ stream_ids, int n_streams,
                                                             const int32_t* __restrict__ n_dev, int n_max,
                                                             float* __restrict__ state, float smooth_coeff) {
   __shared__ float s_R[9];
@@ -32,8 +36,13 @@ __global__ void __launch_bounds__(SM_ELEMS) one_euro_kernel(float* __restrict__ 
   const int n = n_dev ? min(*n_dev, n_max) : n_max;
   if (row >= n) return;
   if (detection_flag && !(detection_flag[row] > 0.f)) return;   // undetected hands are not filtered (main.py:72-79)
-  const int t = hand_type ? (hand_type[row] != 0) : row;
-  float* st = state + (size_t)t * SM_STATE;
+  int bank = hand_type ? (hand_type[row] != 0) : row;
+  if (stream_ids) {
+    const int s = stream_ids[batch_ids[row]];
+    if (s < 0 || s >= n_streams) return;                        // padding slot: no stream, no state touched
+    bank += 2 * s;
+  }
+  float* st = state + (size_t)bank * SM_STATE;
   float* p = poses + (size_t)row * 48;
   float x, mincut;
   if (e < 45) { x = p[3 + e]; mincut = smooth_coeff; }
@@ -75,8 +84,25 @@ extern "C" int acr_b200_one_euro_smooth(float* poses, float* betas, const int32_
   ACR_CHECK_ARG(n_max >= 0 && (n_max == 0 || (poses && betas && state)), "one_euro_smooth: bad arguments");
   ACR_CHECK_ARG(smooth_coeff > 0.f, "one_euro_smooth: smooth_coeff must be positive");
   if (n_max == 0) return ACR_B200_OK;
-  one_euro_kernel<<<n_max, SM_ELEMS, 0, (cudaStream_t)stream>>>(poses, betas, hand_type, detection_flag, n_dev, n_max,
-                                                                state, smooth_coeff);
+  one_euro_kernel<<<n_max, SM_ELEMS, 0, (cudaStream_t)stream>>>(poses, betas, hand_type, detection_flag, nullptr,
+                                                                nullptr, 0, n_dev, n_max, state, smooth_coeff);
+  ACR_CHECK_LAUNCH();
+  return ACR_B200_OK;
+}
+
+extern "C" int acr_b200_one_euro_smooth_streams(float* poses, float* betas, const int32_t* hand_type,
+                                                const float* detection_flag, const int64_t* batch_ids,
+                                                const int32_t* stream_ids, int n_streams, const int32_t* n_dev,
+                                                int n_max, float* state, float smooth_coeff, void* stream) {
+  ACR_CHECK_ARG(n_max >= 0 && n_streams > 0 && (n_max == 0 || (poses && betas && state)),
+                "one_euro_smooth_streams: bad arguments");
+  ACR_CHECK_ARG(n_max == 0 || (hand_type && batch_ids && stream_ids),
+                "one_euro_smooth_streams: hand_type, batch_ids and stream_ids are required");
+  ACR_CHECK_ARG(smooth_coeff > 0.f, "one_euro_smooth_streams: smooth_coeff must be positive");
+  if (n_max == 0) return ACR_B200_OK;
+  one_euro_kernel<<<n_max, SM_ELEMS, 0, (cudaStream_t)stream>>>(poses, betas, hand_type, detection_flag, batch_ids,
+                                                                stream_ids, n_streams, n_dev, n_max, state,
+                                                                smooth_coeff);
   ACR_CHECK_LAUNCH();
   return ACR_B200_OK;
 }

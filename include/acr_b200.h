@@ -137,6 +137,21 @@ size_t acr_b200_one_euro_state_floats(void);
 int acr_b200_one_euro_smooth(float* poses, float* betas, const int32_t* hand_type, const float* detection_flag,
                              const int32_t* n_dev, int n_max, float* state, float smooth_coeff, void* stream);
 
+/* The same filter for many independent video streams in one launch (one row per hand, any number of slots).
+ * `state`: n_streams consecutive blocks of acr_b200_one_euro_state_floats() floats; block s is stream s's
+ * history, laid out exactly like the single-stream state above (zeroing block s on the launching stream
+ * resets stream s: "new clip").  The bank of row r is (stream_ids[batch_ids[r]], hand_type[r]):
+ *   batch_ids (n) int64   slot of each row (acr_b200_parse / _per_frame write it)
+ *   stream_ids (B) int32  stream of each slot; a slot whose id is outside [0, n_streams), e.g. -1 for a
+ *                         padding slot, is not filtered and leaves every state block untouched.
+ * Rows with detection_flag == 0 are skipped as above.  CONTRACT: the non-negative stream ids of one call are
+ * distinct -- two slots of the same stream in one launch would race on its state.  hand_type, batch_ids and
+ * stream_ids are required.  acr_b200_one_euro_smooth is this kernel with one stream and the bank = hand type. */
+int acr_b200_one_euro_smooth_streams(float* poses, float* betas, const int32_t* hand_type,
+                                     const float* detection_flag, const int64_t* batch_ids,
+                                     const int32_t* stream_ids, int n_streams, const int32_t* n_dev, int n_max,
+                                     float* state, float smooth_coeff, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Rotations
  * ---------------------------------------------------------------------------------------- */
@@ -155,7 +170,8 @@ typedef struct acr_b200_map {      /* one fp32 NHWC map: element (b,y,x,c) at   
 } acr_b200_map;
 
 typedef struct acr_b200_parse_out {
-  /* compacted rows, left hands first (all images in order) then right hands; capacity 2*B */
+  /* compacted rows, left hands first (all images in order) then right hands; capacity 2*B
+   * (acr_b200_parse_per_frame: fixed rows, see there)                                     */
   float* params_pred;        /* (2B,109) */
   float* cam;                /* (2B,3)   */
   float* global_orient;      /* (2B,3)   axis-angle */
@@ -173,7 +189,7 @@ typedef struct acr_b200_parse_out {
   /* dense per-image scratch, (B,2): flat index and score of the top-1 centre of each side */
   int32_t* top_idx;
   float* top_score;
-  int32_t* row_src;          /* (2B,4) scratch: image, side, flat index, other side's index | -1 */
+  int32_t* row_src;          /* (2B,4) scratch: image, side (| 2: per-frame dummy row), flat index, other side's index | -1 */
 } acr_b200_parse_out;
 
 /* ResultParser.parse (acr/result_parser.py:21-40) = parse_maps (:85-190) with K=1 centre
@@ -185,6 +201,20 @@ int acr_b200_parse(acr_b200_map l_center, acr_b200_map r_center, acr_b200_map l_
                    acr_b200_map r_params, acr_b200_map l_prior, acr_b200_map r_prior, int B,
                    float conf_thresh, const int64_t* meta_batch_ids, const float* offsets,
                    acr_b200_parse_out out, void* stream);
+
+/* Per-frame parse: every image b is parsed exactly as the reference's ResultParser.parse parses that image
+ * alone (a batch of one), so a row never depends on the other images of the batch -- the semantics of B
+ * independent video streams.  Same arguments and output struct as acr_b200_parse, but a FIXED layout, no
+ * compaction: row b is image b's left hand, row B+b its right hand, counts = [B, B, 2B, #true, #left, #right].
+ *   - a side not detected in image b gets the reference's batch-of-one dummy row: sampled at pixel 0 of
+ *     image b, no prior, detection_flag 0, hand_type = that side, reorganize_idx = meta_batch_ids[b];
+ *   - the cross-hand prior is applied iff image b detected both hands and their centres are at most 32 apart
+ *     on the 64-grid (determine_coeff evaluated on image b).
+ * One thread per image replaces acr_b200_parse's one-CTA batch scan.                                  */
+int acr_b200_parse_per_frame(acr_b200_map l_center, acr_b200_map r_center, acr_b200_map l_params,
+                             acr_b200_map r_params, acr_b200_map l_prior, acr_b200_map r_prior, int B,
+                             float conf_thresh, const int64_t* meta_batch_ids, const float* offsets,
+                             acr_b200_parse_out out, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Network launch plan (backbone + heads)
